@@ -365,6 +365,24 @@ def bench_frame_loop(dev):
             "frame_ms": ms, "ms_per_step": ms / n_iter, "rays_per_s": B * n_frames * n_pix / (ms * 1e-3)}
 
 
+def dump_outputs(out_dir, ens):
+    """What the last timed step hands its caller: the per-object loss terms it computed and the parameters after
+    its AdamW update, one float32 ``<name>.npy`` per array (20 objects at hidden 32: under 1 MB).
+
+    The inputs are the same in every run.  The outputs are only as reproducible as the step: by default the fused
+    kernel sums weight-gradient MMAs in arrival order, and AdamW amplifies that rounding over the run (two runs of
+    ``--steps 200 --warmup 10`` on a B200 at 1000 W: loss terms within ~1e-3 relative, parameters within ~2 % rel-L2).
+    With ``VMB_DETERMINISTIC=1`` the step is bitwise reproducible (tests/test_umma_gpu.py::test_step_is_reproducible),
+    so two builds can be compared bit for bit."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"loss_terms": ens.loss_terms}
+    arrays.update({"params." + k: v for k, v in ens.stacked().items()})
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().float().cpu().numpy())
+    log(f"wrote {len(arrays)} arrays of the last timed step to {out_dir}")
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -447,6 +465,8 @@ def run_ours(args):
     ms_total = max_over_ranks(e0.elapsed_time(e1))
     ens.check_status()
     log(f"device-resident arm: {ms_total / K * 1e3:.1f} us/step")
+    if args.dump_outputs and rank == 0:           # before the arms below take more steps on the same ensemble
+        dump_outputs(args.dump_outputs, ens)
 
     # ---- same steps launched eagerly with CUDA events around the step kernel (roofline) ----
     k1_events = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(K)]
@@ -571,8 +591,15 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-extras", action="store_true", help="skip the configs[4] / drop-in / frame-loop arms")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the loss terms and updated parameters of the last "
+                    "timed step (rank 0's objects) as DIR/<name>.npy; inputs are seeded, and with VMB_DETERMINISTIC=1 "
+                    "so is the result, so runs compare array by array")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs applies to the GPU arm only")
         run_reference(args)
     else:
         run_ours(args)
